@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload h1|h1c|v1|t1|v2] [--batch B]
     python bench.py --impl reference ...      # the CPU restatement (oracle) on the host cores
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's results (see dump_outputs)
 
 A "step" = one pass of the hot path over one batch of B queries through the C ABI
 (oc_search): hybrid = embedding scan + BM25 posting scorer + fusion/top-k.  N_BATCHES distinct
@@ -78,7 +79,14 @@ def parse():
     ap.add_argument("--recall-queries", type=int, default=1024, help="queries of the fp64 recall check")
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip oracle parity, recall and the CPU baseline")
     ap.add_argument("--no-extra", action="store_true", help="skip the configs[1] sub-result of the h1 line")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's results as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200 (the reference leg times a load-dependent sample)")
+    return args
 
 
 def peaks():
@@ -161,7 +169,6 @@ def run_reference(args, w, batch, n_docs):
     built here) on all host cores, each step a bounded sample of the same workload."""
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     import oracle as orc
-    orc.build()
     wl = make_workload(w, n_docs, batch, 0, 1, True)
     cores = os.cpu_count() or 1
     ix = orc.StrIndex(wl["data_all"]) if w["vocab"] else None
@@ -285,6 +292,31 @@ def recall_hits(got_docs, exp_docs, exp_scores, got_scores):
     for d, s in zip(exp_docs, exp_scores):
         hit += (int(d) in g) or abs(s - exp_scores[-1]) <= 1e-6
     return hit, len(exp_docs)
+
+
+DUMP_CAP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, raw):
+    """Writes one step's results, the arrays execute_batch_arrays returns, as out_dir/<name>.npy so that
+    two builds can be compared output for output: doc_ids [B, limit] (float64: ids < 2**53 are exact),
+    scores [B, limit] float32, n [B] and count [B] float64.  Slots past n hold the library's padding (0).
+    When the whole batch exceeds DUMP_CAP_BYTES, a fixed seeded sample of its queries is written and
+    query_index [b] (float64) names the rows kept."""
+    docs, scores, n, cnt = raw
+    B, limit = docs.shape
+    per_query = limit * (8 + 4) + 8 + 8 + 8
+    room = DUMP_CAP_BYTES - 5 * 128          # five .npy headers of 128 bytes
+    rows = np.arange(B)
+    if B * per_query > room:
+        rows = np.sort(np.random.default_rng(0).choice(B, room // per_query, replace=False))
+    out = {"doc_ids": docs[rows].astype(np.float64), "scores": scores[rows].astype(np.float32),
+           "n": n[rows].astype(np.float64), "count": cnt[rows].astype(np.float64)}
+    if rows.size < B:
+        out["query_index"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def main():
@@ -426,6 +458,8 @@ def main():
         return
 
     K, B = args.steps, batch
+    if args.dump_outputs:      # every rank holds the merged answer: rank 0 writes it
+        dump_outputs(args.dump_outputs, last[(K - 1) % N_BATCHES])
     value = B * K / (dev_ms * 1e-3)
     e2e = B * K / (wall_ms * 1e-3)
     pk, peak_src = peaks()
@@ -495,7 +529,6 @@ def main():
     elif check:
         sys.path.insert(0, os.path.join(ROOT, "oracle"))
         import oracle as orc
-        orc.build()
         rows_all = wl.get("rows_all")
         ix = orc.StrIndex(wl["data_all"]) if w["vocab"] else None
         st = orc.EmbStore(rows_all) if w["dim"] else None

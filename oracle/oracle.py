@@ -70,9 +70,11 @@ _lib = None
 
 
 def lib():
+    """Loads the library build() made without recompiling it, so callers such as bench.py never write
+    into the tree; it is compiled here only when it is missing."""
     global _lib
     if _lib is None:
-        L = C.CDLL(build())
+        L = C.CDLL(_SO if os.path.exists(_SO) else build())
         L.orc_idf.restype = C.c_float
         L.orc_idf.argtypes = [C.c_float, C.c_uint64]
         L.orc_normalized_tf.restype = C.c_float

@@ -1,10 +1,11 @@
 """Generates tests/golden/games_fulltext.npz — BASELINE configs[0], "benches/fulltext_simple.rs on
 games.json": the reference's own CPU-runnable plumbing case.
 
-Run in the build container (reads /root/reference/benches/games.json, which does not exist on the GPU
-box).  The fixture holds only DERIVED integer / float arrays — the committed postings of the 1512 game
-documents (fields title, description) as laid out by oramacore_b200.hostindex (lower-case alphanumeric
-tokenizer; the reference's stemmer lives in an un-vendored crate), the resolved term lists of a query
+    python tests/golden/make_games_fixture.py <oramacore checkout>/benches/games.json
+
+The tests read only the fixture, never games.json.  The fixture holds only DERIVED integer / float
+arrays — the committed postings of the 1512 game documents (fields title, description) as laid out
+by oramacore_b200.hostindex (lower-case alphanumeric tokenizer; the reference's stemmer lives in an un-vendored crate), the resolved term lists of a query
 set (the bench's own strings + game-domain ones, prefix and exact resolution), and the ORACLE's answers
 (count, top-10 doc ids and scores).  tests/test_gpu_zz_games_config0.py checks the oracle against the stored
 answers on the CPU and the GPU path against the oracle on a B200."""
@@ -28,7 +29,7 @@ QUERIES = [  # (term, exact, on the GPU test too?)  benches/fulltext_simple.rs:4
 
 
 def main():
-    games = json.load(open("/root/reference/benches/games.json"))
+    games = json.load(open(sys.argv[1]))
     h = HostStringIndex(("title", "description"))
     for i, g in enumerate(games):
         h.insert(i, {"title": g.get("title", ""), "description": g.get("description", "")})

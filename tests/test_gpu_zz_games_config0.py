@@ -1,8 +1,8 @@
 """BASELINE configs[0] — "benches/fulltext_simple.rs on games.json (CPU-only reference, plumbing)":
 fulltext search over the 1512 game documents (fields title + description) for the bench's own query
 strings and a few game-domain ones.  The corpus travels as a derived fixture (committed postings +
-resolved query terms + the oracle's answers; tests/golden/make_games_fixture.py), because
-/root/reference does not exist on the GPU box."""
+resolved query terms + the oracle's answers; tests/golden/make_games_fixture.py), so the test needs
+nothing outside the repository."""
 import os
 
 import numpy as np
