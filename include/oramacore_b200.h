@@ -249,6 +249,38 @@ int oc_facets_add_number_field(oc_facets *f, uint64_t n, const double *values_so
 int oc_search_facets(oc_ctx *ctx, oc_emb *emb, oc_str *str, oc_facets *facets, const oc_search_params *p,
                      const oc_facet_req *reqs, uint32_t n_reqs, uint64_t *out_counts);
 
+/* ---- sortBy over the score map -----------------------------------------------------------------------
+ * sort_token_scores with Some(sort_by) (read/sort.rs:17-98, 236-257): instead of the relevance top-n, the score map's
+ * keys in the order of a number, date or bool field — value groups in the requested order (IndexSortContext::execute,
+ * read/index/sort.rs:186-264), ascending DocumentId inside a group — then skip(offset).take(limit).  Each hit carries
+ * its score-map value.  The score map is exactly oc_search's: where-filter, uncommitted deletes, threshold, OMC and
+ * hybrid fusion apply, and out_count is oc_search's count.  A document without a value in the field is never emitted
+ * but still counts.  Number values compare as f64 (NaN rejected), dates as exact i64, bools false < true.  A document
+ * may hold one value per field (listing it twice is OC_ERR_INVALID).  A store is immutable once built: to refresh it,
+ * build a new one.  nbits: DocumentId space [0, nbits), at most 2^32. */
+typedef struct oc_sort oc_sort;            /* == the bool / number / date field storages IndexSortContext reads */
+int oc_sort_create(oc_ctx *ctx, uint64_t nbits, oc_sort **out);
+void oc_sort_destroy(oc_sort *s);
+int oc_sort_add_number_field(oc_sort *s, uint64_t n, const uint64_t *doc_ids, const double *values, uint32_t *out_field);
+int oc_sort_add_date_field(oc_sort *s, uint64_t n, const uint64_t *doc_ids, const int64_t *ts, uint32_t *out_field);
+int oc_sort_add_bool_field(oc_sort *s, uint64_t n_true, const uint64_t *true_docs, uint64_t n_false, const uint64_t *false_docs,
+                           uint32_t *out_field);
+/* Outputs as oc_search; out_keys: NULL or B x limit, the sort value of each hit (bool: 0 / 1, date: the timestamp as
+ * f64).  An unknown field is OC_ERR_INVALID (SortFieldNotFound); p->sharded is OC_ERR_UNSUPPORTED.  OC_SORT_FORM=walk |
+ * gather forces one of the two device selection forms (otherwise each query picks one from its count). */
+int oc_search_sorted(oc_ctx *ctx, oc_emb *emb, oc_str *str, oc_sort *s, uint32_t field, int descending,
+                     const oc_search_params *p, uint64_t *out_doc_ids, float *out_scores, uint32_t *out_n,
+                     uint64_t *out_count, double *out_keys);
+/* The selection form (0 = walk, 1 = gather) each query of the last oc_search_sorted on ctx took; n_queries <= its B. */
+int oc_sort_last_forms(oc_ctx *ctx, uint32_t n_queries, uint8_t *out);
+/* Multi-index union in field order (MergeSortedIterator, read/sort.rs:491-560), host only, like oc_merge_results:
+ * per index the rows of oc_search_sorted with limit' = limit+offset, offset' = 0, vector_limit = limit and their
+ * out_keys.  Equal keys: the lower index first.  Keys compare exactly (the reference clamps date keys to i32). */
+int oc_merge_sorted_results(uint32_t n_indexes, uint32_t n_queries, uint32_t limit, uint32_t offset, uint32_t in_stride,
+                            int descending, const uint64_t *const *doc_ids, const float *const *scores,
+                            const double *const *keys, const uint32_t *const *n, const uint64_t *const *counts,
+                            uint64_t *out_doc_ids, float *out_scores, uint32_t *out_n, uint64_t *out_count);
+
 /* ---- multi-index collections ---------------------------------------------------------------------
  * search_on_indexes runs every index of a collection into ONE score map (read/search.rs:304-338,
  * token_score.rs:472-499): document ids are unique per collection, so the per-index maps are disjoint; hybrid

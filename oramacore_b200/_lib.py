@@ -27,6 +27,8 @@ EXPORTED_SYMBOLS = [
     "oc_filter_from_ids", "oc_filter_from_bits", "oc_filter_and", "oc_filter_or", "oc_filter_not", "oc_filter_count",
     "oc_filter_read", "oc_filter_destroy", "oc_merge_results",
     "oc_facets_create", "oc_facets_destroy", "oc_facets_add_field", "oc_facets_add_number_field", "oc_search_facets",
+    "oc_sort_create", "oc_sort_destroy", "oc_sort_add_number_field", "oc_sort_add_date_field", "oc_sort_add_bool_field",
+    "oc_search_sorted", "oc_sort_last_forms", "oc_merge_sorted_results",
     "oc_dict_create", "oc_dict_destroy", "oc_dict_add_terms", "oc_dict_lookup", "oc_dict_size", "oc_dict_set_stemmer", "oc_stem_english",
     "oc_dict_resolve", "oc_resolved_arrays", "oc_resolved_fill", "oc_resolved_free",
 ]
@@ -161,6 +163,15 @@ def lib():
     L.oc_facets_add_number_field.argtypes = [vp, u64, vp, vp, C.POINTER(u32)]
     L.oc_search_facets.argtypes = [vp, vp, vp, vp, C.POINTER(SearchParams), C.POINTER(FacetReq), u32, vp]
     L.oc_merge_results.argtypes = [u32, u32, u32, u32, u32, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), vp, vp, vp, vp]
+    L.oc_sort_create.argtypes = [vp, u64, C.POINTER(vp)]
+    L.oc_sort_destroy.argtypes = [vp]
+    L.oc_sort_destroy.restype = None
+    L.oc_sort_add_number_field.argtypes = [vp, u64, vp, vp, C.POINTER(u32)]
+    L.oc_sort_add_date_field.argtypes = [vp, u64, vp, vp, C.POINTER(u32)]
+    L.oc_sort_add_bool_field.argtypes = [vp, u64, vp, u64, vp, C.POINTER(u32)]
+    L.oc_search_sorted.argtypes = [vp, vp, vp, vp, u32, i32, C.POINTER(SearchParams), vp, vp, vp, vp, vp]
+    L.oc_sort_last_forms.argtypes = [vp, u32, vp]
+    L.oc_merge_sorted_results.argtypes = [u32, u32, u32, u32, u32, i32] + [C.POINTER(vp)] * 5 + [vp, vp, vp, vp]
     L.oc_dict_create.argtypes = [u32, C.POINTER(vp)]
     L.oc_dict_destroy.argtypes = [vp]
     L.oc_dict_destroy.restype = None

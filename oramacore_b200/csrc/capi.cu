@@ -23,6 +23,7 @@
 #include "emb_gemm.cuh"
 #include "emb_scan.cuh"
 #include "fuse.cuh"
+#include "sort.cuh"
 #include "oramacore_b200.h"
 
 using namespace oc;
@@ -126,7 +127,7 @@ static bool is_pinned_host(const void *p) {
     return a.type == cudaMemoryTypeHost;
 }
 
-enum { EV_START, EV_H2D, EV_DEV, EV_D2H, EV_SCAN0, EV_SCAN1, EV_BM0, EV_BM1, EV_FUSE0, EV_FUSE1, EV_COMM0, EV_COMM1, EV_SWEEP0, EV_SWEEP1, EV_RR0, EV_RR1, EV_N };
+enum { EV_START, EV_H2D, EV_DEV, EV_D2H, EV_SCAN0, EV_SCAN1, EV_BM0, EV_BM1, EV_FUSE0, EV_FUSE1, EV_COMM0, EV_COMM1, EV_SWEEP0, EV_SWEEP1, EV_RR0, EV_RR1, EV_SORT0, EV_SORT1, EV_N };
 
 constexpr size_t P2P_WIN_BYTES = size_t(1) << 20;   // per (parity, source rank): a batch's records must fit (256 queries x 520 B = 133 KB)
 constexpr uint32_t P2P_MAX_Q = 4096;
@@ -152,6 +153,8 @@ struct oc_ctx {
     DevBuf in_blob, in_blob0, q_pad, q_inv, eff_norm, filter_dev, scan_cand, v_doc, v_score, v_row, v_cnt, v_srow, v_ft, v_present, v_raw;
     DevBuf seg, df_dev, row_ok, tau, cand_key, cand_ft, cand_cnt, tile_cnt, tile_max, tile_min, min_hint;
     DevBuf out_blob, shard_send, shard_recv, work_ctr, flat_desc, mbits, dbits, facet_req, facet_out;
+    DevBuf sort_pick, sort_npick, sort_form, sort_rows, sort_ft, sort_present, sort_max, sort_keys;
+    std::vector<uint8_t> sort_forms;  // SORT_FORM_* of each query of the last oc_search_sorted
     bool gemm_pending = false; const float *gemm_inv_norm = nullptr;
     DevBuf q_bf16, q_rho, pre_post, dense_buf, g_thr, g_eps, g_ovf, g_ovfcnt, g_resc, g_cand, g_cnt, g_flag, g_max, r_qpad, r_qinv, r_map, r_doc, r_score, r_row, r_cnt, r_raw;
 
@@ -207,7 +210,8 @@ extern "C" void oc_shutdown(oc_ctx *c) {
                       &c->v_score, &c->v_row, &c->v_cnt, &c->v_srow, &c->v_ft, &c->v_present, &c->v_raw, &c->seg, &c->df_dev,
                       &c->row_ok, &c->tau, &c->cand_key, &c->cand_ft, &c->cand_cnt, &c->tile_cnt, &c->tile_max,
                       &c->tile_min, &c->min_hint, &c->out_blob, &c->shard_send, &c->shard_recv, &c->work_ctr, &c->flat_desc, &c->mbits, &c->dbits, &c->facet_req, &c->facet_out, &c->q_bf16, &c->q_rho, &c->pre_post, &c->dense_buf, &c->g_thr, &c->g_eps, &c->g_ovf, &c->g_ovfcnt, &c->g_resc, &c->g_cand, &c->g_cnt, &c->g_max,
-                      &c->g_flag, &c->r_qpad, &c->r_qinv, &c->r_map, &c->r_doc, &c->r_score, &c->r_row, &c->r_cnt, &c->r_raw};
+                      &c->g_flag, &c->r_qpad, &c->r_qinv, &c->r_map, &c->r_doc, &c->r_score, &c->r_row, &c->r_cnt, &c->r_raw,
+                      &c->sort_pick, &c->sort_npick, &c->sort_form, &c->sort_rows, &c->sort_ft, &c->sort_present, &c->sort_max, &c->sort_keys};
     for (DevBuf *b : bufs) b->release();
     c->h_in.release(); c->h_out.release();
     for (int i = 0; i < EV_N; i++) if (c->ev[i]) cudaEventDestroy(c->ev[i]);
@@ -1230,6 +1234,7 @@ extern "C" int oc_str_info(oc_str *s, oc_str_info_t *out) {
 
 // ------------------------------------------------------------------------------------ device-resident filters
 struct oc_facets;
+struct oc_sort;
 struct oc_filter {
     oc_ctx *ctx;
     uint64_t nbits, words;
@@ -1541,9 +1546,18 @@ struct FacetJob {   // oc_search_facets: count, per query, the matched documents
 };
 static int run_facets(oc_ctx *c, const FacetJob &fj, uint32_t B, bool has_ft, bool has_v, const StrSnap *S, uint32_t n_tiles,
                       uint32_t vlimit);
+struct SortJob {    // oc_search_sorted: replace the top-n by the first limit+offset score-map keys in a field's order
+    oc_sort *st;
+    uint32_t field;
+    bool descending;
+    int form;           // SORT_FORM_* (OC_SORT_FORM)
+    double *out_keys;   // NULL or [B][limit]
+};
+static int run_sort(oc_ctx *c, const SortJob &sj, const oc_search_params *p, uint32_t B, bool has_ft, bool has_v, const StrSnap *S,
+                    uint32_t n_tiles, uint32_t vlimit, uint32_t n_keep, const FuseParams &fp, const Bm25Params &bp, const uint32_t *row_ok);
 
 static int search_impl(oc_ctx *c, oc_emb *emb, oc_str *str, const oc_search_params *p, uint64_t *out_doc_ids,
-                       float *out_scores, uint32_t *out_n, uint64_t *out_count, const FacetJob *fj) {
+                       float *out_scores, uint32_t *out_n, uint64_t *out_count, const FacetJob *fj, const SortJob *sj) {
     if (!c || !p || !out_doc_ids || !out_scores || !out_n || !out_count) return fail(OC_ERR_INVALID, "NULL argument");
     const uint32_t B = p->n_queries;
     if (B == 0) return OC_OK;
@@ -1961,7 +1975,7 @@ static int search_impl(oc_ctx *c, oc_emb *emb, oc_str *str, const oc_search_para
                 off += cls_nq[g] * n_tiles; q0 += cls_nq[g];
             }
         }
-        if (fj) {   // facets: the tile kernels also emit the bitmap of matched rows (every (query, tile) item writes its 256 words)
+        if (fj || sj) {   // facets / sortBy: the tile kernels also emit the bitmap of matched rows (every (query, tile) item writes its 256 words)
             OCTRY(c->mbits.ensure(size_t(B) * std::max<uint32_t>(n_tiles, 1) * (BM25_TILE / 32) * 4));
             bp.matched_bits = c->mbits.as<uint32_t>();
         }
@@ -2023,6 +2037,10 @@ static int search_impl(oc_ctx *c, oc_emb *emb, oc_str *str, const oc_search_para
     fp.out_doc = reinterpret_cast<uint64_t *>(dout + o_doc); fp.out_score = reinterpret_cast<float *>(dout + o_sc);
     fp.out_n = reinterpret_cast<uint32_t *>(dout + o_n); fp.out_count = reinterpret_cast<unsigned long long *>(dout + o_cnt);
     fp.out_min = reinterpret_cast<float *>(dout + o_min);
+    if (sj) {
+        OCTRY(c->sort_max.ensure(size_t(B) * 4));
+        fp.out_max = c->sort_max.as<float>();
+    }
     fuse_smem = size_t(fp.capb) * 8 + size_t(std::max<uint32_t>(32, next_pow2(n_keep))) * 8 + size_t(vlimit) * 8 + 64;
     if (smem_cfg_needed(c->device, (const void *)fuse_topk_kernel, fuse_smem))
         CU(cudaFuncSetAttribute(fuse_topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fuse_smem));
@@ -2094,17 +2112,32 @@ static int search_impl(oc_ctx *c, oc_emb *emb, oc_str *str, const oc_search_para
         }
     }
     if (fj) OCTRY(run_facets(c, *fj, B, has_ft, has_v, S, n_tiles, vlimit));
+    float sort_ms = 0.f;
+    if (sj) {   // after every re-run: the bitmap, the count and K4's extrema are final
+        CU(cudaEventRecord(c->ev[EV_SORT0], c->stream));
+        OCTRY(run_sort(c, *sj, p, B, has_ft, has_v, S, n_tiles, vlimit, n_keep, fp, bp, row_ok));
+        CU(cudaEventRecord(c->ev[EV_SORT1], c->stream));
+        CU(cudaMemcpyAsync(h, dout, out_bytes, cudaMemcpyDeviceToHost, c->stream));
+        if (sj->out_keys) CU(cudaMemcpyAsync(sj->out_keys, c->sort_keys.p, size_t(B) * p->limit * 8, cudaMemcpyDeviceToHost, c->stream));
+        c->sort_forms.resize(B);
+        CU(cudaMemcpyAsync(c->sort_forms.data(), c->sort_form.p, B, cudaMemcpyDeviceToHost, c->stream));
+        CU(cudaStreamSynchronize(c->stream));
+        CU(cudaEventElapsedTime(&sort_ms, c->ev[EV_SORT0], c->ev[EV_SORT1]));
+    }
     c->timing.d2h_bytes = out_bytes;
     memcpy(out_doc_ids, h + o_doc, size_t(B) * p->limit * 8);
     memcpy(out_scores, h + o_sc, size_t(B) * p->limit * 4);
     memcpy(out_n, h + o_n, size_t(B) * 4);
     memcpy(out_count, h + o_cnt, size_t(B) * 8);
-    return finish_timing(c, has_v && emb->n_rows > 0, has_ft, true, did_comm);
+    OCTRY(finish_timing(c, has_v && emb->n_rows > 0, has_ft, true, did_comm));
+    c->timing.device_ms += sort_ms;   // the sortBy kernels run after the plain tail's events
+    c->timing.fuse_ms += sort_ms;
+    return OC_OK;
 }
 
 extern "C" int oc_search(oc_ctx *c, oc_emb *emb, oc_str *str, const oc_search_params *p, uint64_t *out_doc_ids,
                          float *out_scores, uint32_t *out_n, uint64_t *out_count) {
-    return search_impl(c, emb, str, p, out_doc_ids, out_scores, out_n, out_count, nullptr);
+    return search_impl(c, emb, str, p, out_doc_ids, out_scores, out_n, out_count, nullptr, nullptr);
 }
 
 // ------------------------------------------------------------------------------------ facets
@@ -2236,6 +2269,39 @@ __global__ void __launch_bounds__(256) facet_count_kernel(const FacetReqDev *req
     }
 }
 
+// the key set of each query's score map as a DocumentId bitmap over [0, *cap_bits): the tile scorers' matched rows
+// (c->mbits) + the vector hits; *stride in u32 words
+static int score_map_bits(oc_ctx *c, uint32_t B, bool has_ft, bool has_v, const StrSnap *S, uint32_t n_tiles, uint32_t vlimit,
+                          uint64_t nbits, const uint32_t **bits, uint64_t *stride, uint64_t *cap_bits) {
+    const uint64_t row_words = uint64_t(n_tiles) * (BM25_TILE / 32);
+    const uint64_t doc_words = (nbits + 31) / 32;
+    const bool identity = has_ft && S->row_doc == nullptr;
+    if (identity && !has_v) {   // the row bitmap is the document bitmap
+        *bits = c->mbits.as<uint32_t>(); *stride = row_words; *cap_bits = S->n_rows;
+        return OC_OK;
+    }
+    OCTRY(c->dbits.ensure(size_t(B) * doc_words * 4));
+    CU(cudaMemsetAsync(c->dbits.p, 0, size_t(B) * doc_words * 4, c->stream));
+    if (has_ft && n_tiles) {
+        if (identity) {
+            const uint64_t wcopy = std::min(row_words, doc_words);
+            CU(cudaMemcpy2DAsync(c->dbits.p, doc_words * 4, c->mbits.p, row_words * 4, wcopy * 4, B, cudaMemcpyDeviceToDevice, c->stream));
+        } else {
+            dim3 grid((unsigned)((row_words + 255) / 256), B);
+            facet_rows_to_docs_kernel<<<grid, 256, 0, c->stream>>>(c->mbits.as<uint32_t>(), row_words, S->row_doc, S->n_rows,
+                                                                  c->dbits.as<uint32_t>(), doc_words, nbits);
+            launched(c);
+        }
+    }
+    if (has_v) {
+        facet_mark_hits_kernel<<<(B * vlimit + 255) / 256, 256, 0, c->stream>>>(c->v_doc.as<uint64_t>(), c->v_cnt.as<uint32_t>(), vlimit, B,
+                                                                              c->dbits.as<uint32_t>(), doc_words, nbits);
+        launched(c);
+    }
+    *bits = c->dbits.as<uint32_t>(); *stride = doc_words; *cap_bits = nbits;
+    return OC_OK;
+}
+
 static int run_facets(oc_ctx *c, const FacetJob &fj, uint32_t B, bool has_ft, bool has_v, const StrSnap *S, uint32_t n_tiles,
                       uint32_t vlimit) {
     oc_facets *fc = fj.fc;
@@ -2258,34 +2324,8 @@ static int run_facets(oc_ctx *c, const FacetJob &fj, uint32_t B, bool has_ft, bo
         rd[i].docs = fl.docs + lo; rd[i].n = hi - lo;
         max_n = std::max(max_n, rd[i].n);
     }
-    // the key set of each query's score map as a DocumentId bitmap
-    const uint64_t row_words = uint64_t(n_tiles) * (BM25_TILE / 32);
-    const uint64_t doc_words = (fc->nbits + 31) / 32;
-    const bool identity = has_ft && S->row_doc == nullptr;
-    const uint32_t *bits; uint64_t stride, cap_bits;
-    if (identity && !has_v) {   // the row bitmap is the document bitmap
-        bits = c->mbits.as<uint32_t>(); stride = row_words; cap_bits = S->n_rows;
-    } else {
-        OCTRY(c->dbits.ensure(size_t(B) * doc_words * 4));
-        CU(cudaMemsetAsync(c->dbits.p, 0, size_t(B) * doc_words * 4, c->stream));
-        if (has_ft && n_tiles) {
-            if (identity) {
-                const uint64_t wcopy = std::min(row_words, doc_words);
-                CU(cudaMemcpy2DAsync(c->dbits.p, doc_words * 4, c->mbits.p, row_words * 4, wcopy * 4, B, cudaMemcpyDeviceToDevice, c->stream));
-            } else {
-                dim3 grid((unsigned)((row_words + 255) / 256), B);
-                facet_rows_to_docs_kernel<<<grid, 256, 0, c->stream>>>(c->mbits.as<uint32_t>(), row_words, S->row_doc, S->n_rows,
-                                                                      c->dbits.as<uint32_t>(), doc_words, fc->nbits);
-                launched(c);
-            }
-        }
-        if (has_v) {
-            facet_mark_hits_kernel<<<(B * vlimit + 255) / 256, 256, 0, c->stream>>>(c->v_doc.as<uint64_t>(), c->v_cnt.as<uint32_t>(), vlimit, B,
-                                                                                  c->dbits.as<uint32_t>(), doc_words, fc->nbits);
-            launched(c);
-        }
-        bits = c->dbits.as<uint32_t>(); stride = doc_words; cap_bits = fc->nbits;
-    }
+    const uint32_t *bits = nullptr; uint64_t stride = 0, cap_bits = 0;
+    OCTRY(score_map_bits(c, B, has_ft, has_v, S, n_tiles, vlimit, fc->nbits, &bits, &stride, &cap_bits));
     OCTRY(c->facet_req.ensure(size_t(fj.n_reqs) * sizeof(FacetReqDev)));
     OCTRY(c->facet_out.ensure(size_t(B) * fj.n_reqs * 8));
     CU(cudaMemcpyAsync(c->facet_req.p, rd.data(), size_t(fj.n_reqs) * sizeof(FacetReqDev), cudaMemcpyHostToDevice, c->stream));
@@ -2317,7 +2357,222 @@ extern "C" int oc_search_facets(oc_ctx *c, oc_emb *emb, oc_str *str, oc_facets *
     std::vector<float> scores(size_t(B) * p->limit);
     std::vector<uint32_t> n(B);
     FacetJob fj{facets, reqs, n_reqs, out_counts};
-    return search_impl(c, emb, str, &q, docs.data(), scores.data(), n.data(), cnt.data(), &fj);
+    return search_impl(c, emb, str, &q, docs.data(), scores.data(), n.data(), cnt.data(), &fj, nullptr);
+}
+
+// ------------------------------------------------------------------------------------ sortBy
+// sort_token_scores with Some(sort_by) (read/sort.rs:17-98, 236-257): the first limit+offset keys of the score map in
+// the order IndexSortContext::execute yields (read/index/sort.rs:186-264), each with its score-map value.  Per field
+// the store keeps on the device a dense rank of every document's value (SORT_NONE = no value), the two walk orders
+// (rank ascending / descending, DocumentId ascending inside a rank) and the value of each rank (out_keys).
+struct SortField {
+    uint32_t *rank = nullptr;                       // device [nbits]
+    uint32_t *order_asc = nullptr, *order_desc = nullptr;   // device [n_pop] DocumentIds
+    double *rank_value = nullptr;                   // device [n_ranks]
+    uint64_t n_pop = 0;
+    uint32_t n_ranks = 0;
+};
+struct oc_sort {
+    oc_ctx *ctx;
+    uint64_t nbits;                                 // DocumentId space [0, nbits)
+    std::vector<SortField> fields;
+};
+
+extern "C" int oc_sort_create(oc_ctx *c, uint64_t nbits, oc_sort **out) {
+    if (!c || !out || nbits == 0) return fail(OC_ERR_INVALID, "bad arguments");
+    if (nbits > (uint64_t(1) << 32)) return fail(OC_ERR_UNSUPPORTED, "sort store: nbits %llu > 2^32", (unsigned long long)nbits);
+    oc_sort *s = new oc_sort();
+    s->ctx = c; s->nbits = nbits;
+    *out = s;
+    return OC_OK;
+}
+static void sort_field_free(SortField &f) {
+    cudaFree(f.rank); cudaFree(f.order_asc); cudaFree(f.order_desc); cudaFree(f.rank_value);
+    f = SortField{};
+}
+extern "C" void oc_sort_destroy(oc_sort *s) {
+    if (!s) return;
+    {
+        std::lock_guard<std::mutex> g(s->ctx->mu);
+        cudaSetDevice(s->ctx->device);
+        cudaStreamSynchronize(s->ctx->stream);
+        for (auto &f : s->fields) sort_field_free(f);
+    }
+    delete s;
+}
+// (doc, key) pairs -> ranks and walk orders.  Key: double (number), int64 (date, exact), uint8 (bool: false < true).
+template <typename K>
+static int sort_add(oc_sort *s, uint64_t n, const uint64_t *docs, const K *keys, uint32_t *out_field) {
+    std::vector<uint64_t> idx(n);
+    for (uint64_t i = 0; i < n; i++) {
+        if (docs[i] >= s->nbits) return fail(OC_ERR_INVALID, "sort field: document %llu >= nbits", (unsigned long long)docs[i]);
+        idx[i] = i;
+    }
+    std::sort(idx.begin(), idx.end(), [&](uint64_t a, uint64_t b) { return keys[a] < keys[b] || (keys[a] == keys[b] && docs[a] < docs[b]); });
+    std::vector<uint32_t> rank(s->nbits, SORT_NONE), asc(n), desc(n);
+    std::vector<double> value;
+    std::vector<uint64_t> group;   // start of each rank's run in asc
+    for (uint64_t j = 0; j < n; j++) {
+        const uint64_t i = idx[j];
+        if (j == 0 || keys[i] != keys[idx[j - 1]]) { value.push_back(double(keys[i])); group.push_back(j); }
+        // the reference would emit such a document once per value (an array field): not representable in one rank
+        if (rank[docs[i]] != SORT_NONE) return fail(OC_ERR_INVALID, "sort field: document %llu is listed twice", (unsigned long long)docs[i]);
+        rank[docs[i]] = uint32_t(value.size() - 1);
+        asc[j] = uint32_t(docs[i]);
+    }
+    group.push_back(n);
+    for (size_t g = group.size() - 1, o = 0; g-- > 0;)   // ranks descending, DocumentId ascending inside a rank
+        for (uint64_t j = group[g]; j < group[g + 1]; j++) desc[o++] = asc[j];
+    oc_ctx *c = s->ctx;
+    std::lock_guard<std::mutex> g(c->mu);
+    CU(cudaSetDevice(c->device));
+    SortField f;
+    f.n_pop = n; f.n_ranks = uint32_t(value.size());
+    auto up = [&](void **dst, const void *src, size_t bytes) -> int {
+        cudaError_t e = cudaMalloc(dst, std::max<size_t>(bytes, 8));
+        if (e != cudaSuccess) return fail(OC_ERR_OOM, "cudaMalloc(sort field): %s", cudaGetErrorString(e));
+        if (bytes) CU(cudaMemcpy(*dst, src, bytes, cudaMemcpyHostToDevice));
+        return OC_OK;
+    };
+    int rc = up(reinterpret_cast<void **>(&f.rank), rank.data(), rank.size() * 4);
+    if (rc == OC_OK) rc = up(reinterpret_cast<void **>(&f.order_asc), asc.data(), n * 4);
+    if (rc == OC_OK) rc = up(reinterpret_cast<void **>(&f.order_desc), desc.data(), n * 4);
+    if (rc == OC_OK) rc = up(reinterpret_cast<void **>(&f.rank_value), value.data(), value.size() * 8);
+    if (rc != OC_OK) { sort_field_free(f); return rc; }
+    s->fields.push_back(f);
+    if (out_field) *out_field = uint32_t(s->fields.size() - 1);
+    return OC_OK;
+}
+extern "C" int oc_sort_add_number_field(oc_sort *s, uint64_t n, const uint64_t *doc_ids, const double *values, uint32_t *out_field) {
+    if (!s || (n && (!doc_ids || !values))) return fail(OC_ERR_INVALID, "bad arguments");
+    for (uint64_t i = 0; i < n; i++) if (values[i] != values[i]) return fail(OC_ERR_INVALID, "sort field: value %llu is NaN", (unsigned long long)i);
+    return sort_add(s, n, doc_ids, values, out_field);
+}
+extern "C" int oc_sort_add_date_field(oc_sort *s, uint64_t n, const uint64_t *doc_ids, const int64_t *ts, uint32_t *out_field) {
+    if (!s || (n && (!doc_ids || !ts))) return fail(OC_ERR_INVALID, "bad arguments");
+    return sort_add(s, n, doc_ids, ts, out_field);
+}
+extern "C" int oc_sort_add_bool_field(oc_sort *s, uint64_t n_true, const uint64_t *true_docs, uint64_t n_false, const uint64_t *false_docs,
+                                      uint32_t *out_field) {
+    if (!s || (n_true && !true_docs) || (n_false && !false_docs)) return fail(OC_ERR_INVALID, "bad arguments");
+    std::vector<uint64_t> docs(false_docs, false_docs + n_false);
+    docs.insert(docs.end(), true_docs, true_docs + n_true);
+    std::vector<uint8_t> keys(n_false, 0);
+    keys.resize(n_false + n_true, 1);
+    return sort_add(s, docs.size(), docs.data(), keys.data(), out_field);
+}
+
+static int run_sort(oc_ctx *c, const SortJob &sj, const oc_search_params *p, uint32_t B, bool has_ft, bool has_v, const StrSnap *S,
+                    uint32_t n_tiles, uint32_t vlimit, uint32_t n_keep, const FuseParams &fp, const Bm25Params &bp, const uint32_t *row_ok) {
+    const SortField &fl = sj.st->fields[sj.field];
+    SortSelParams sp{};
+    OCTRY(score_map_bits(c, B, has_ft, has_v, S, n_tiles, vlimit, sj.st->nbits, &sp.bits, &sp.stride_words, &sp.cap_bits));
+    OCTRY(c->sort_pick.ensure(size_t(B) * n_keep * 8));
+    OCTRY(c->sort_npick.ensure(size_t(B) * 4));
+    OCTRY(c->sort_form.ensure(B));
+    OCTRY(c->sort_keys.ensure(size_t(B) * p->limit * 8));
+    sp.count = fp.out_count;
+    sp.rank = fl.rank; sp.nbits = sj.st->nbits;
+    sp.order = sj.descending ? fl.order_desc : fl.order_asc;
+    sp.n_pop = fl.n_pop; sp.n_ranks = fl.n_ranks; sp.descending = sj.descending ? 1 : 0;
+    sp.n_keep = n_keep; sp.form = sj.form;
+    sp.pick = c->sort_pick.as<uint64_t>(); sp.n_pick = c->sort_npick.as<uint32_t>(); sp.form_out = c->sort_form.as<uint8_t>();
+    const size_t smem = (size_t(SORT_GATHER_CAP) + std::max<uint32_t>(32, next_pow2(n_keep))) * 8;
+    if (smem_cfg_needed(c->device, (const void *)sort_select_kernel, smem))
+        CU(cudaFuncSetAttribute(sort_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    sort_select_kernel<<<B, SORT_THREADS, smem, c->stream>>>(sp);
+    launched(c);
+    CU(cudaGetLastError());
+    SortScoreParams ss{};
+    if (has_ft) {   // the fulltext score of every pick: the point lookups of the hybrid path (bm25_point_kernel)
+        OCTRY(c->sort_rows.ensure(size_t(B) * n_keep * 4));
+        OCTRY(c->sort_ft.ensure(size_t(B) * n_keep * 4));
+        OCTRY(c->sort_present.ensure(size_t(B) * n_keep));
+        map_docs_to_rows_kernel<<<(B * n_keep + 255) / 256, 256, 0, c->stream>>>(sp.pick, sp.n_pick, n_keep, B, S->row_doc, S->n_rows,
+                                                                                c->sort_rows.as<uint32_t>());
+        launched(c);
+        PointParams pp{};
+        pp.terms = bp.terms; pp.tokens = bp.tokens; pp.queries = bp.queries;
+        pp.n_queries = B; pp.v_stride = n_keep; pp.v_row = c->sort_rows.as<uint32_t>(); pp.row_ok_bits = row_ok;
+        pp.k = p->bm25_k; pp.threshold = p->threshold >= 0.0f ? 1 : 0;
+        pp.v_ft = c->sort_ft.as<float>(); pp.v_present = c->sort_present.as<uint8_t>();
+        bm25_point_kernel<<<(unsigned)((uint64_t(B) * n_keep * 32 + 255) / 256), 256, 0, c->stream>>>(pp);
+        launched(c);
+        CU(cudaGetLastError());
+        ss.p_ft = pp.v_ft; ss.p_present = pp.v_present;
+    }
+    ss.fp = fp; ss.n_queries = B;
+    ss.gmin = fp.out_min; ss.gmax = fp.out_max;
+    ss.pick = sp.pick; ss.n_pick = sp.n_pick;
+    ss.rank = fl.rank; ss.rank_value = fl.rank_value;
+    ss.out_key = c->sort_keys.as<double>();
+    sort_score_kernel<<<(unsigned)((uint64_t(B) * p->limit + 255) / 256), 256, 0, c->stream>>>(ss);
+    launched(c);
+    CU(cudaGetLastError());
+    return OC_OK;
+}
+
+extern "C" int oc_search_sorted(oc_ctx *c, oc_emb *emb, oc_str *str, oc_sort *s, uint32_t field, int descending,
+                                const oc_search_params *p, uint64_t *out_doc_ids, float *out_scores, uint32_t *out_n,
+                                uint64_t *out_count, double *out_keys) {
+    if (!c || !p || !s) return fail(OC_ERR_INVALID, "NULL argument");
+    if (s->ctx != c) return fail(OC_ERR_INVALID, "sort store belongs to another ctx");
+    if (p->sharded) return fail(OC_ERR_UNSUPPORTED, "sortBy over a sharded search: sort per shard and merge with oc_merge_sorted_results");
+    if (field >= s->fields.size()) return fail(OC_ERR_INVALID, "unknown sort field %u", field);   // SortFieldNotFound
+    const char *fe = getenv("OC_SORT_FORM");   // walk | gather: force one selection form (A/B runs, tests)
+    const int form = (fe && !strcmp(fe, "walk")) ? SORT_FORM_WALK : (fe && !strcmp(fe, "gather")) ? SORT_FORM_GATHER : SORT_FORM_AUTO;
+    SortJob sj{s, field, descending != 0, form, out_keys};
+    return search_impl(c, emb, str, p, out_doc_ids, out_scores, out_n, out_count, nullptr, &sj);
+}
+
+extern "C" int oc_sort_last_forms(oc_ctx *c, uint32_t n_queries, uint8_t *out) {
+    if (!c || (n_queries && !out)) return fail(OC_ERR_INVALID, "NULL argument");
+    std::lock_guard<std::mutex> g(c->mu);
+    if (n_queries > c->sort_forms.size()) return fail(OC_ERR_INVALID, "the last sorted search had %zu queries", c->sort_forms.size());
+    if (n_queries) memcpy(out, c->sort_forms.data(), n_queries);
+    return OC_OK;
+}
+
+// MergeSortedIterator (read/sort.rs:491-560) + truncate over per-index lists already in field order: the list whose head
+// key comes first wins; on equal keys the lower index wins (its whole value group comes first, as the iterator's strict
+// comparison yields it).  Keys are compared exactly (dates too: no i32 clamp).
+extern "C" int oc_merge_sorted_results(uint32_t n_indexes, uint32_t B, uint32_t limit, uint32_t offset, uint32_t in_stride,
+                                       int descending, const uint64_t *const *doc_ids, const float *const *scores,
+                                       const double *const *keys, const uint32_t *const *n, const uint64_t *const *counts,
+                                       uint64_t *out_doc_ids, float *out_scores, uint32_t *out_n, uint64_t *out_count) {
+    if (!doc_ids || !scores || !keys || !n || !counts || !out_doc_ids || !out_scores || !out_n || !out_count)
+        return fail(OC_ERR_INVALID, "NULL argument");
+    if (limit == 0) return fail(OC_ERR_INVALID, "limit must be >= 1");
+    std::vector<uint32_t> head(n_indexes);
+    for (uint32_t q = 0; q < B; q++) {
+        std::fill(head.begin(), head.end(), 0u);
+        uint64_t cnt = 0;
+        for (uint32_t i = 0; i < n_indexes; i++) {
+            if (n[i][q] > in_stride) return fail(OC_ERR_INVALID, "index %u query %u: n > in_stride", i, q);
+            cnt += counts[i][q];
+        }
+        uint32_t taken = 0, written = 0;
+        while (written < limit) {
+            int best = -1;
+            for (uint32_t i = 0; i < n_indexes; i++) {
+                if (head[i] >= n[i][q]) continue;
+                if (best < 0) { best = (int)i; continue; }
+                const double ka = keys[i][size_t(q) * in_stride + head[i]], kb = keys[best][size_t(q) * in_stride + head[best]];
+                if (descending ? ka > kb : ka < kb) best = (int)i;
+            }
+            if (best < 0) break;
+            if (taken >= offset) {
+                out_doc_ids[size_t(q) * limit + written] = doc_ids[best][size_t(q) * in_stride + head[best]];
+                out_scores[size_t(q) * limit + written] = scores[best][size_t(q) * in_stride + head[best]];
+                written++;
+            }
+            taken++; head[best]++;
+        }
+        for (uint32_t k = written; k < limit; k++) { out_doc_ids[size_t(q) * limit + k] = 0; out_scores[size_t(q) * limit + k] = 0.f; }
+        out_n[q] = written;
+        out_count[q] = cnt;
+    }
+    return OC_OK;
 }
 
 // ------------------------------------------------------------------------------------ micro-batching front

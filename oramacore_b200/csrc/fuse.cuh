@@ -44,6 +44,7 @@ struct FuseParams {
     uint32_t *out_n;
     unsigned long long *out_count;
     float *out_min;               // actual global min (rank-proxy validation), may be NULL
+    float *out_max;               // actual global max (sortBy re-scores picked documents with it), may be NULL
 };
 
 __device__ __forceinline__ float omc_lookup(const FuseParams &p, uint64_t doc, bool *found) {
@@ -222,6 +223,7 @@ __global__ void __launch_bounds__(256) fuse_topk_kernel(const FuseParams p) {
         p.out_n[q] = n_out;
         p.out_count[q] = s_count;
         if (p.out_min) p.out_min[q] = gmin;
+        if (p.out_max) p.out_max[q] = gmax;
     }
 }
 

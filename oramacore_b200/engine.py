@@ -408,6 +408,108 @@ def search_facets(tsc: "TokenScoreContext", store: FacetStore, params: "TokenSco
     return res
 
 
+class SortStore:
+    """The bool / number / date fields of one Index laid out for sortBy on the device (oc_sort_*): per field a dense
+    rank of every document's value and the two walk orders of IndexSortContext::execute (read/index/sort.rs:186-264).
+    Immutable once built: to refresh it, build a new one."""
+
+    def __init__(self, ctx: Context, nbits: int):
+        self.ctx, self.nbits = ctx, int(nbits)
+        self._h = C.c_void_p()
+        check(lib().oc_sort_create(ctx._h, self.nbits, C.byref(self._h)))
+        self.fields: Dict[str, int] = {}
+
+    def _add(self, name: str, fn, *args) -> int:
+        fid = C.c_uint32()
+        check(fn(self._h, *args, C.byref(fid)))
+        self.fields[name] = fid.value
+        return fid.value
+
+    def add_number_field(self, name: str, doc_ids, values) -> int:
+        """One number per document (i64 and f64 values compare as f64, number_field.rs:466-549); NaN is rejected."""
+        d = np.ascontiguousarray(doc_ids, np.uint64)
+        v = np.ascontiguousarray(values, np.float64)
+        assert d.shape == v.shape
+        return self._add(name, lib().oc_sort_add_number_field, d.shape[0], _p(d), _p(v))
+
+    def add_date_field(self, name: str, doc_ids, timestamps) -> int:
+        """One i64 timestamp per document, compared exactly (date_field.rs:239-246)."""
+        d = np.ascontiguousarray(doc_ids, np.uint64)
+        t = np.ascontiguousarray(timestamps, np.int64)
+        assert d.shape == t.shape
+        return self._add(name, lib().oc_sort_add_date_field, d.shape[0], _p(d), _p(t))
+
+    def add_bool_field(self, name: str, true_docs, false_docs) -> int:
+        """false before true ascending (index/sort.rs:210-241)."""
+        t = np.ascontiguousarray(true_docs, np.uint64)
+        f = np.ascontiguousarray(false_docs, np.uint64)
+        return self._add(name, lib().oc_sort_add_bool_field, t.shape[0], _p(t), f.shape[0], _p(f))
+
+    def close(self):
+        if self._h:
+            lib().oc_sort_destroy(self._h)
+            self._h = None
+
+
+def _sort_order(sort_by: dict) -> bool:
+    """SortBy {property, order}: order defaults to ASC (types.rs:1351-1364); returns descending."""
+    order = sort_by.get("order", "ASC")
+    if order not in ("ASC", "DESC"):
+        raise ValueError(f"sortBy order must be ASC or DESC, got {order!r}")
+    return order == "DESC"
+
+
+def search_sorted(tsc: "TokenScoreContext", store: SortStore, params: "TokenScoreParams", sort_by: dict, texts=None,
+                  q_vecs: Optional[np.ndarray] = None, with_keys: bool = False):
+    """sort_token_scores with Some(sort_by) (read/sort.rs:17-98): per query the score map's keys in the order of
+    sort_by["property"], skip(offset).take(limit), each with its score-map value; count as execute_batch.  An unknown
+    property raises KeyError (SortFieldNotFound).  with_keys: also return, per query, the sort value of each hit."""
+    prop = sort_by["property"]
+    if prop not in store.fields:
+        raise KeyError(f"sort field not found: {prop!r}")
+    desc = _sort_order(sort_by)
+    sp, keep, B = tsc._build_params(params, texts, q_vecs)
+    L = params.limit_hint
+    docs, scores = np.empty((B, L), np.uint64), np.empty((B, L), np.float32)
+    n, cnt, keys = np.empty(B, np.uint32), np.empty(B, np.uint64), np.empty((B, L), np.float64)
+    check(lib().oc_search_sorted(tsc.ctx._h, tsc.emb._h if tsc.emb else None, tsc.str._h if tsc.str else None, store._h,
+                                 store.fields[prop], int(desc), C.byref(sp), _p(docs), _p(scores), _p(n), _p(cnt), _p(keys)))
+    hits = [SearchHits(docs[i, :n[i]].copy(), scores[i, :n[i]].copy(), int(cnt[i])) for i in range(B)]
+    if with_keys:
+        return hits, [keys[i, :n[i]].copy() for i in range(B)]
+    return hits
+
+
+def sort_last_forms(ctx: Context, n_queries: int) -> np.ndarray:
+    """The selection form (0 = walk, 1 = gather) each query of the last search_sorted on ctx took."""
+    out = np.zeros(max(n_queries, 1), np.uint8)
+    check(lib().oc_sort_last_forms(ctx._h, int(n_queries), _p(out)))
+    return out[:n_queries]
+
+
+def merge_sorted_index_results(per_index, limit: int, offset: int = 0, order: str = "ASC") -> List[SearchHits]:
+    """The multi-index union in field order (MergeSortedIterator, read/sort.rs:491-560) + skip/take: per_index = one
+    (hits, keys) pair per index as search_sorted(..., with_keys=True) returns it, each run with
+    limit_hint = limit+offset, offset = 0, vector_limit = limit.  count = the sum of the per-index counts."""
+    k = len(per_index)
+    B = len(per_index[0][0])
+    stride = max(1, max(len(h.doc_ids) for hits, _ in per_index for h in hits))
+    keep = []
+    for hits, keys in per_index:
+        d, s_, kk = np.zeros((B, stride), np.uint64), np.zeros((B, stride), np.float32), np.zeros((B, stride), np.float64)
+        n, c = np.zeros(B, np.uint32), np.zeros(B, np.uint64)
+        for q, h in enumerate(hits):
+            m = len(h.doc_ids)
+            d[q, :m], s_[q, :m], kk[q, :m], n[q], c[q] = h.doc_ids, h.scores, keys[q], m, h.count
+        keep.append([d, s_, kk, n, c])
+    arr = lambda j: (C.c_void_p * k)(*[r[j].ctypes.data for r in keep])
+    od, os_ = np.zeros((B, limit), np.uint64), np.zeros((B, limit), np.float32)
+    on, oc = np.zeros(B, np.uint32), np.zeros(B, np.uint64)
+    check(lib().oc_merge_sorted_results(k, B, limit, offset, stride, int(_sort_order({"order": order})), arr(0), arr(1), arr(2),
+                                        arr(3), arr(4), _p(od), _p(os_), _p(on), _p(oc)))
+    return [SearchHits(od[i, :on[i]].copy(), os_[i, :on[i]].copy(), int(oc[i])) for i in range(B)]
+
+
 def merge_index_results(per_index, limit: int, offset: int = 0) -> List[SearchHits]:
     """search_on_indexes' union of the per-index score maps + top_n + skip/take (search.rs:304-338, 482-498):
     per_index = one (doc_ids [B, limit+offset], scores, n, count) tuple per index, each obtained with

@@ -14,6 +14,7 @@ use std::ffi::{c_char, c_int, c_void, CStr};
 #[repr(C)] pub struct OcBatcher { _p: [u8; 0] }
 #[repr(C)] pub struct OcFilter { _p: [u8; 0] }
 #[repr(C)] pub struct OcFacets { _p: [u8; 0] }
+#[repr(C)] pub struct OcSort { _p: [u8; 0] }
 #[repr(C)] pub struct OcDict { _p: [u8; 0] }
 #[repr(C)] pub struct OcResolved { _p: [u8; 0] }
 
@@ -131,6 +132,22 @@ extern "C" {
                             doc_ids: *const *const u64, scores: *const *const f32, n: *const *const u32,
                             counts: *const *const u64, out_doc_ids: *mut u64, out_scores: *mut f32,
                             out_n: *mut u32, out_count: *mut u64) -> c_int;
+    // sortBy over the score map (read/sort.rs:17-98, index/sort.rs:186-264)
+    pub fn oc_sort_create(ctx: *mut OcCtx, nbits: u64, out: *mut *mut OcSort) -> c_int;
+    pub fn oc_sort_destroy(s: *mut OcSort);
+    pub fn oc_sort_add_number_field(s: *mut OcSort, n: u64, doc_ids: *const u64, values: *const f64, out_field: *mut u32) -> c_int;
+    pub fn oc_sort_add_date_field(s: *mut OcSort, n: u64, doc_ids: *const u64, ts: *const i64, out_field: *mut u32) -> c_int;
+    pub fn oc_sort_add_bool_field(s: *mut OcSort, n_true: u64, true_docs: *const u64, n_false: u64, false_docs: *const u64,
+                                  out_field: *mut u32) -> c_int;
+    pub fn oc_search_sorted(ctx: *mut OcCtx, emb: *mut OcEmb, s: *mut OcStr, st: *mut OcSort, field: u32, descending: c_int,
+                            p: *const OcSearchParams, out_doc_ids: *mut u64, out_scores: *mut f32, out_n: *mut u32,
+                            out_count: *mut u64, out_keys: *mut f64) -> c_int;
+    pub fn oc_sort_last_forms(ctx: *mut OcCtx, n_queries: u32, out: *mut u8) -> c_int;
+    /// MergeSortedIterator (read/sort.rs:491-560) over per-index sorted rows, host side
+    pub fn oc_merge_sorted_results(n_indexes: u32, n_queries: u32, limit: u32, offset: u32, in_stride: u32, descending: c_int,
+                                   doc_ids: *const *const u64, scores: *const *const f32, keys: *const *const f64,
+                                   n: *const *const u32, counts: *const *const u64, out_doc_ids: *mut u64, out_scores: *mut f32,
+                                   out_n: *mut u32, out_count: *mut u64) -> c_int;
     // term dictionary + batch query resolution (tokenize_and_stem + FST expansion), host only
     pub fn oc_dict_create(n_fields: u32, out: *mut *mut OcDict) -> c_int;
     pub fn oc_dict_destroy(d: *mut OcDict);
